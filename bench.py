@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
   python bench.py --impl reference --gpus N --steps K ...  # reference arithmetic on the host CPU cores
+  python bench.py ... --dump-outputs DIR                   # also write the last timed step's outputs as DIR/<name>.npy
 
 A "step" is one full training pass of the hot path over one synthetic batch: Model.call (fused input gather +
 two-stream U-Net + UV->camera tail), L2 loss, full backward to every weight gradient, (N>1: the gradient all-reduce
@@ -255,7 +256,12 @@ class TrainRun:
         for i in range(max(warmup, 3)):
             self.step(self.resident[i % 2])
         l0, tc0 = nat.launch_count(), nat.tc_launch_count()
-        ms = timed(self.strategy, lambda i: self.step(self.resident[i % 2]), steps, self.dev)
+        last = {}
+
+        def fn(i):
+            last['out'] = self.step(self.resident[i % 2])
+        ms = timed(self.strategy, fn, steps, self.dev)
+        self.last_out = last['out']
         launches, tc = nat.launch_count() - l0, nat.tc_launch_count() - tc0
         if self.graphed is not None and self.graphed.graph is not None:
             # replayed kernels are not seen by the library's counter: add the captured ones per replay
@@ -311,6 +317,45 @@ class TrainRun:
         summ = engine.PROF.summary()
         engine.PROF.enabled = False
         return summ
+
+    def outputs(self):
+        """What the last timed step handed its caller: the loss and the tensors the model computed for `to_vis`
+        (inputs passed through are left out), plus the parameters after its update and its weight gradients, each
+        of the latter flattened in sorted parameter-name order of the Keras layout."""
+        loss, to_vis = self.last_out
+        params, grads = self.model.export_params(), self.model.export_grads()
+        out = {'loss': loss}
+        out.update((k, to_vis[k]) for k in ('pred', 'pred_camspc', 'base_camspc', 'gt_camspc'))
+        out['params'] = torch.cat([params[k].reshape(-1) for k in sorted(params)])
+        out['grads'] = torch.cat([grads[k].reshape(-1) for k in sorted(grads)])
+        return out
+
+
+DUMP_SAMPLE = 1 << 21          # elements kept of a larger output (8 MB in float32); at most 7 outputs are written
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """`--dump-outputs`: every array as <out_dir>/<name>.npy, float64 kept and anything else as float32, so that two
+    builds can be compared output for output.  An array of more than DUMP_SAMPLE elements is replaced by a fixed
+    sample of its flattened elements: one per stride of size // DUMP_SAMPLE, at an offset drawn from a generator
+    seeded with 0, in ascending index order (the same positions on every run and every build)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, t in arrays.items():
+        a = t.detach()
+        a = a if a.dtype == torch.float64 else a.float()
+        n = a.numel()
+        if n > DUMP_SAMPLE:
+            stride = n // DUMP_SAMPLE
+            off = torch.randint(stride, (DUMP_SAMPLE,), generator=torch.Generator().manual_seed(0))
+            a = a.reshape(-1)[(torch.arange(DUMP_SAMPLE) * stride + off).to(a.device)]
+        a = a.cpu().numpy()
+        total += a.nbytes
+        if total > DUMP_LIMIT:
+            raise SystemExit('bench.py: --dump-outputs would exceed %d bytes at %s' % (DUMP_LIMIT, name))
+        np.save(os.path.join(out_dir, name + '.npy'), a)
 
 
 def parity_check(run):
@@ -372,7 +417,7 @@ def measure_tf32_peak(dev):
     return 2.0 * n ** 3 / (best * 1e-3) / 1e12
 
 
-def forward_record(strategy, wl, batch, steps, warmup):
+def forward_record(strategy, wl, batch, steps, warmup, dump_dir=None):
     """cfg1: forward only (mode 'test') through the cached observation features, device-resident and end to end."""
     import models
     import nlt_native as nat
@@ -389,8 +434,15 @@ def forward_record(strategy, wl, batch, steps, warmup):
     for i in range(max(warmup, 3)):
         model.call(resident[i % 2], 'test', obs_override=feat)
     l0 = nat.launch_count()
-    ms = timed(strategy, lambda i: model.call(resident[i % 2], 'test', obs_override=feat), steps, dev)
+    last = {}
+
+    def fwd(i):
+        last['out'] = model.call(resident[i % 2], 'test', obs_override=feat)
+    ms = timed(strategy, fwd, steps, dev)
     launches = nat.launch_count() - l0
+    if dump_dir is not None and strategy.rank == 0:
+        pred_c, _, _, to_vis = last['out']
+        dump_outputs(dump_dir, {'pred_camspc': pred_c, 'pred': to_vis['pred'], 'base_camspc': to_vis['base_camspc']})
 
     def e2e(i):
         b = tuple(t.to(dev, non_blocking=True) if torch.is_tensor(t) else t for t in host[i % 2])
@@ -472,7 +524,7 @@ def run_b200(args):
     global_bs = batch * world
 
     if not wl['train']:
-        rec = forward_record(strategy, wl, batch, args.steps, args.warmup)
+        rec = forward_record(strategy, wl, batch, args.steps, args.warmup, args.dump_outputs)
         if rank == 0:
             emit({'metric': 'UV texels/sec fwd', 'value': rec['value'], 'unit': UNIT, 'n_gpus': world,
                   'steps': args.steps, 'warmup': max(args.warmup, 3), 'ms_per_step': rec['ms_per_step'],
@@ -493,6 +545,8 @@ def run_b200(args):
         sampler.start()
     ms_step, launches, tc_launches = run.measure_resident(args.steps, 0)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, run.outputs())
 
     # ---- end-to-end arm ----
     ms_e2e, h2d_bytes = run.measure_e2e(args.steps)
@@ -646,9 +700,15 @@ def main():
     ap.add_argument('--no-parity', action='store_true', help='skip the in-bench parity gate')
     ap.add_argument('--no-graph', dest='no_graph', action='store_true', help='launch kernels eagerly (no CUDA graph)')
     ap.add_argument('--profile-out', dest='profile_out', default=None, help='write the per-op device-time table here')
+    ap.add_argument('--dump-outputs', dest='dump_outputs', default=None, metavar='DIR',
+                    help='after the timed steps, write what the last one computed as DIR/<name>.npy (rank 0)')
     ap.add_argument('--sub', default=None, help=argparse.SUPPRESS)
     ap.add_argument('--sub-timeout', dest='sub_timeout', type=int, default=240, help=argparse.SUPPRESS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and (args.impl != 'b200' or args.sub):
+        ap.error('--dump-outputs writes the outputs of the B200 path (--impl b200)')
     _guard_stdout()
     if args.impl == 'reference':
         run_reference(args)

@@ -34,8 +34,10 @@ def _worker(rank, world, port, q):
     for p in (ROOT, os.path.join(ROOT, 'neural-light-transport_b200')):
         if p not in sys.path:
             sys.path.insert(0, p)
+    # the ranks compute on the CPU: with a GPU visible, Strategy would bind rank r to cuda:r, which a machine with
+    # fewer GPUs than ranks does not have
     os.environ.update(RANK=str(rank), WORLD_SIZE=str(world), LOCAL_RANK=str(rank), MASTER_ADDR='127.0.0.1',
-                      MASTER_PORT=str(port))
+                      MASTER_PORT=str(port), CUDA_VISIBLE_DEVICES='')
     import trainvali
     from oracle import nlt_oracle as O
     from util import synth

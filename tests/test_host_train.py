@@ -53,8 +53,9 @@ def _reducer_worker(rank, world, port, q):
     for p in (ROOT, os.path.join(ROOT, 'neural-light-transport_b200')):
         if p not in sys.path:
             sys.path.insert(0, p)
+    # CPU-only ranks (see tests/test_dist.py): no rank may bind a GPU that a one-GPU machine does not have
     os.environ.update(RANK=str(rank), WORLD_SIZE=str(world), LOCAL_RANK=str(rank), MASTER_ADDR='127.0.0.1',
-                      MASTER_PORT=str(port))
+                      MASTER_PORT=str(port), CUDA_VISIBLE_DEVICES='')
     import engine
     import trainvali
     torch.set_num_threads(1)
